@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — consensus records/s on schema S32 (BASELINE.json `metric`), device-resident and end-to-end.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--n 16] [--records 1000000] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--n 16] [--records 1000000] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch: K1 (vote, 24 fields) + K2 (numeric, 8 fields) over
 `records` records per GPU with n candidates (BASELINE configs[1]: 1M x 32 fields, n=16); at N > 1 every rank owns
@@ -268,6 +268,31 @@ def bind_to_gpu_numa_node(gpu_index: int):
     return None
 
 
+DUMP_RECORDS = 1 << 16  # 512 B per record as float64: 32 MiB in all
+
+
+def dump_outputs(out_dir, n_records, win, vmeta, value, nmeta):
+    """Write this rank's results of the last timed step as float64 .npy files: the winning code and result word of every
+    vote field, the value and result word of every numeric field, for a fixed sample of records (all of them up to
+    DUMP_RECORDS; beyond, a seeded sample in record order, listed in records.npy).  float64 holds every int32 code and
+    uint32 word exactly, so two builds can be compared bit for bit."""
+    import numpy as np
+    import torch
+    idx = np.arange(n_records)
+    if n_records > DUMP_RECORDS:
+        idx = np.sort(np.random.default_rng(0).choice(n_records, DUMP_RECORDS, replace=False))
+    rows = torch.from_numpy(idx).to(win.device)
+    pick = lambda t: t.view(n_records, -1)[rows].cpu().numpy()  # noqa: E731
+    arrays = {"records": idx.astype(np.float64),
+              "vote_win_code": pick(win).astype(np.float64),
+              "vote_meta": pick(vmeta).view(np.uint32).astype(np.float64),
+              "numeric_value": pick(value),
+              "numeric_meta": pick(nmeta).view(np.uint32).astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_gpu_arm(args):
     import numpy as np
     import torch
@@ -500,9 +525,11 @@ def run_gpu_arm(args):
             lw, lm = fused.local_win, fused.local_vmeta
             expect = (lw & 0x3FFFF) | (((lm >> 6) & 0x7F) << 18) | (((lm >> 20) & 0x7F) << 25)
             assert torch.equal(win, expect), "packed gathered vote words differ from the local full results"
-            win = lw
+            win, vmeta = lw, lm
     else:
         win, vmeta, value, nmeta = [torch.cat([sharded.my_views(c)[k] for c in range(chunks)]) for k in range(4)]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, N, win, vmeta, value, nmeta)
 
     # --- end to end, the reference's unit of work: candidate JSON texts (pinned host memory) -> consensus / likelihoods texts
     e2e = None
@@ -701,7 +728,13 @@ def main():
     ap.add_argument("--sweep", default="", help="comma-separated candidate counts, e.g. 2,4,8,16,32,64: one JSON line per n (configs[4])")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the last step's results (a seeded sample of records) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.sweep or args.impl == "reference"):
+        ap.error("--dump-outputs takes the results of one GPU run: not with --sweep or --impl reference")
     args.sweep_push_mode, args.sweep_push_chunks = args.push_mode, args.push_chunks
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.gpus != world and world == 1 and args.gpus > 1 and args.impl == "b200":
