@@ -213,6 +213,34 @@ int kc_weighted_vote_i32(const int32_t *d_codes, const float *d_seq_logprob, int
                          void *stream);
 
 /*
+ * Candidate weights of likelihood-weighted consolidation (NEW feature, self-defined: DESIGN.md §5) — K3b's weight pre-pass:
+ *   d_seq_logprob float32[n_records][n]  ->  d_weight float32[n_records][n],  w_c = kexp(s_c - max_k s_k) per record
+ * (kexp: the fixed-order fp32 exp of K3b).  1 <= n <= 64.  A slot that is not a candidate of its record can be filled with
+ * -3.0e38f: it never raises the record's maximum.
+ */
+int kc_candidate_weights_f32(const float *d_seq_logprob, int64_t n_records, int32_t n, float *d_weight, void *stream);
+
+/*
+ * Likelihood-weighted vote over IRREGULAR groups (NEW feature, self-defined: DESIGN.md §5): K3b's vote (class weight = fp32 sum of
+ * its cells' weights in cell order; the heaviest class wins; among equal weights the class whose first cell comes first) for
+ * groups that need not be fields of one fixed record layout.
+ *   d_cells        [n_groups][n]  K1's coding (code >= 0 class, KC_CODE_NONE, < KC_CODE_NONE absent); None cells do not vote
+ *                  (int8: the device JSON path's cell matrix, int32: the planner's)
+ *   d_group_record int32[n_groups]  the record of each group (index into d_weight's rows)
+ *   d_cand         int8[n_groups][n] or NULL: the candidate of each present cell (NULL: cell c is candidate c)
+ *   d_weight       float32[n_records][n] (kc_candidate_weights_f32)
+ *   d_meta         uint32[n_groups]  K1's result word: idx | support | nn | present | flags; KC_FLAG_TIE when another class
+ *                  weighs exactly as much as the winner
+ *   d_sums         float32[n_groups][2] (8-byte aligned): W_win (0 if no cell voted), W_present = fp32 sum of the weights of the
+ *                  present cells, None cells included, in cell order.  Confidence: round(pvf * (W_win / W_present), 5) in double.
+ * 1 <= n <= 64.
+ */
+int kc_weighted_vote_groups_i8(const int8_t *d_cells, int64_t n_groups, int32_t n, const int32_t *d_group_record, const int8_t *d_cand,
+                               const float *d_weight, uint32_t *d_meta, float *d_sums, void *stream);
+int kc_weighted_vote_groups_i32(const int32_t *d_cells, int64_t n_groups, int32_t n, const int32_t *d_group_record, const int8_t *d_cand,
+                                const float *d_weight, uint32_t *d_meta, float *d_sums, void *stream);
+
+/*
  * K4 — similarity medoid of string groups (consensus_as_primitive fallback, consensus_utils.py:1221-1237, with
  * levenshtein_similarity :745-761): pairwise 1 - dist/max_len (floored at 1e-8) on NORMALISED strings (lower-case [a-z0-9],
  * normalize_string :660-673, done by the caller), np.nanmean of each row in numpy's summation order, first argmax.
@@ -339,6 +367,18 @@ typedef struct {
 } kc_json_stats;
 int kc_consolidate_json_packed(const char *h_text, const int64_t *h_off, int64_t n_records, int32_t n, double rel_eps, double abs_eps,
                                int device, int32_t threads, uint32_t flags, kc_json_result **out);
+/*
+ * H1g with the likelihood-weighted vote (NEW feature, self-defined: DESIGN.md §5).  The arguments of kc_consolidate_json_packed plus
+ *   h_lp      float32 token logprobs of every candidate, back to back
+ *   h_lp_off  int64[n_records * n + 1]  candidate c of record r has the tokens h_lp[h_lp_off[r*n+c] .. h_lp_off[r*n+c+1]) (ascending)
+ * Per chunk the logprobs go to the device next to the texts; K3 sums them per candidate, kc_candidate_weights_f32 turns the sums
+ * into weights, and the vote fields are decided by kc_weighted_vote_groups_i8 (confidence round(W_win / W_present, 5)).  Numeric
+ * and multi-word fields are not weighted.  The host path H1 does not weight: records the device path declines keep status 1 (as
+ * with KC_JSON_DEVICE_ONLY).  stats.input_bytes counts the logprob bytes.
+ */
+int kc_consolidate_json_packed_weighted(const char *h_text, const int64_t *h_off, const float *h_lp, const int64_t *h_lp_off,
+                                        int64_t n_records, int32_t n, double rel_eps, double abs_eps, int device, int32_t threads,
+                                        uint32_t flags, kc_json_result **out);
 /* record r: content = text[content_off[r] .. +content_len[r]), likelihoods likewise; `why` = the device path's reason code for
  * declining (0 = not declined; kc_jsoncore.cuh D_*).  Pointers stay valid until kc_json_result_free.  Any output may be NULL. */
 int kc_json_result_view(kc_json_result *res, const char **text, const int64_t **content_off, const int64_t **content_len,
@@ -359,6 +399,12 @@ int kc_debug_jsongpu_emit(kc_debug_jsongpu *h, const uint32_t *vote_meta, const 
 int kc_debug_jsongpu_medoid_inputs(const kc_debug_jsongpu *h, const uint8_t **chars, const int32_t **str_off, const int32_t **grp_off,
                                    int64_t *n_groups);
 int kc_debug_jsongpu_set_medoid(kc_debug_jsongpu *h, const int32_t *medoid_idx, const double *medoid_avg);
+/* the weighted entry's phases (self-defined, DESIGN.md §5): the record of every vote group (kc_weighted_vote_groups_i8's
+ * d_group_record), and the emit with the weighted vote's float32[n_vote_groups][2] (W_win, W_present) */
+int kc_debug_jsongpu_vote_records(const kc_debug_jsongpu *h, const int32_t **vote_records);
+int kc_debug_jsongpu_emit_weighted(kc_debug_jsongpu *h, const uint32_t *vote_meta, const float *vote_sums, const double *num_value,
+                                   const uint32_t *num_meta, const char **content, const int64_t **content_off, const char **likelihoods,
+                                   const int64_t **likelihoods_off);
 void kc_debug_jsongpu_free(kc_debug_jsongpu *h);
 int kc_debug_parse_doubles(const char *text, const int64_t *off, int64_t count, double *out, uint8_t *ok);
 int kc_debug_float_reprs(const double *xs, int64_t count, char *out /* [count][32] */, int32_t *lens);

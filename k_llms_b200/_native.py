@@ -28,6 +28,8 @@ EXPORTS = (
     "kc_confidence_f64", "kc_logprob_sum_f32", "kc_weighted_vote_i32", "kc_consensus_host", "kc_host_alloc", "kc_host_free",
     "kc_consolidate_json_packed", "kc_json_result_view", "kc_json_result_free", "kc_debug_jsongpu_plan", "kc_debug_jsongpu_inputs",
     "kc_debug_jsongpu_emit", "kc_debug_jsongpu_medoid_inputs", "kc_debug_jsongpu_set_medoid", "kc_debug_jsongpu_free", "kc_debug_parse_doubles", "kc_debug_float_reprs", "kc_debug_round5", "kc_debug_s32_texts", "kc_push_results", "kc_vote_i32_wire", "kc_medoid_str_method",
+    "kc_candidate_weights_f32", "kc_weighted_vote_groups_i8", "kc_weighted_vote_groups_i32", "kc_consolidate_json_packed_weighted",
+    "kc_debug_jsongpu_vote_records", "kc_debug_jsongpu_emit_weighted",
 )
 
 
@@ -64,6 +66,12 @@ def load() -> ctypes.CDLL:
     lib.kc_confidence_f64.argtypes = [vp, i64, i32, vp, vp, vp]
     lib.kc_logprob_sum_f32.argtypes = [vp, vp, i64, vp, vp]
     lib.kc_weighted_vote_i32.argtypes = [vp, vp, i64, i32, i32, vp, vp, vp, vp, vp]
+    lib.kc_candidate_weights_f32.argtypes = [vp, i64, i32, vp, vp]
+    lib.kc_weighted_vote_groups_i8.argtypes = [vp, i64, i32, vp, vp, vp, vp, vp, vp]
+    lib.kc_weighted_vote_groups_i32.argtypes = lib.kc_weighted_vote_groups_i8.argtypes
+    lib.kc_consolidate_json_packed_weighted.argtypes = [vp, vp, vp, vp, i64, i32, f64, f64, c.c_int, i32, c.c_uint32, c.POINTER(vp)]
+    lib.kc_debug_jsongpu_vote_records.argtypes = [vp, c.POINTER(vp)]
+    lib.kc_debug_jsongpu_emit_weighted.argtypes = [vp, vp, vp, vp, vp] + [c.POINTER(vp)] * 4
     lib.kc_consensus_host.argtypes = [vp, i32, vp, vp, i32, i64, i32, f64, f64, vp, vp, vp, vp, c.c_int, vp]
     lib.kc_consensus_host_i8.argtypes = lib.kc_consensus_host.argtypes
     lib.kc_vote_i8.argtypes = [vp, i64, i32, vp, i32, vp, vp, vp]
@@ -115,7 +123,9 @@ def load() -> ctypes.CDLL:
     lib.kc_push_results.restype = c.c_int
     lib.kc_vote_i32_wire.argtypes = [vp, i64, i32, vp, i32, vp, vp, vp, i32, i32, vp, vp, vp]
     lib.kc_vote_i32_wire.restype = c.c_int
-    for name in ("kc_consolidate_json_packed", "kc_json_result_view", "kc_debug_jsongpu_plan", "kc_debug_jsongpu_inputs",
+    for name in ("kc_consolidate_json_packed", "kc_consolidate_json_packed_weighted", "kc_debug_jsongpu_vote_records",
+                 "kc_debug_jsongpu_emit_weighted", "kc_candidate_weights_f32", "kc_weighted_vote_groups_i8", "kc_weighted_vote_groups_i32",
+                 "kc_json_result_view", "kc_debug_jsongpu_plan", "kc_debug_jsongpu_inputs",
                  "kc_debug_jsongpu_emit", "kc_debug_parse_doubles", "kc_debug_float_reprs", "kc_debug_round5"):
         getattr(lib, name).restype = c.c_int
     lib.kc_host_alloc.argtypes = [c.c_uint64]
@@ -244,6 +254,40 @@ def weighted_vote(codes, seq_logprob, none_code=None, stream=None):
     check(load().kc_weighted_vote_i32(codes.data_ptr(), seq_logprob.data_ptr(), R, F, n, nc, win.data_ptr(), meta.data_ptr(),
                                       weight.data_ptr(), _stream_ptr(torch, stream)))
     return win, meta, weight
+
+
+def candidate_weights(seq_logprob, stream=None):
+    """Candidate weights of likelihood-weighted consolidation (self-defined, DESIGN.md §5): seq_logprob float32 [R, n] (cuda) ->
+    float32 [R, n], w_c = kexp(s_c - max_k s_k) per record (K3b's weight pre-pass)."""
+    torch = _require_cuda()
+    assert seq_logprob.is_cuda and seq_logprob.dtype == torch.float32 and seq_logprob.dim() == 2 and seq_logprob.is_contiguous()
+    R, n = seq_logprob.shape
+    out = torch.empty(R, n, dtype=torch.float32, device=seq_logprob.device)
+    _bind(torch, seq_logprob)
+    check(load().kc_candidate_weights_f32(seq_logprob.data_ptr(), R, n, out.data_ptr(), _stream_ptr(torch, stream)))
+    return out
+
+
+def weighted_vote_groups(cells, group_record, weight, cand=None, stream=None):
+    """Likelihood-weighted vote over irregular groups (self-defined, DESIGN.md §5).  cells int8 or int32 [G, n] (K1's coding),
+    group_record int32 [G], weight float32 [R, n] (candidate_weights), cand int8 [G, n] or None (cell c is candidate c); all cuda.
+    Returns (meta int32 [G] holding K1's packed uint32 word, sums float32 [G, 2] = (W_win, W_present))."""
+    torch = _require_cuda()
+    assert cells.is_cuda and cells.dtype in (torch.int8, torch.int32) and cells.dim() == 2 and cells.is_contiguous()
+    G, n = cells.shape
+    assert group_record.is_cuda and group_record.dtype == torch.int32 and group_record.numel() == G and group_record.is_contiguous()
+    assert weight.is_cuda and weight.dtype == torch.float32 and weight.dim() == 2 and weight.shape[1] == n and weight.is_contiguous()
+    cp = None
+    if cand is not None:
+        assert cand.is_cuda and cand.dtype == torch.int8 and tuple(cand.shape) == (G, n) and cand.is_contiguous()
+        cp = cand.data_ptr()
+    meta = torch.empty(G, dtype=torch.int32, device=cells.device)
+    sums = torch.empty(G, 2, dtype=torch.float32, device=cells.device)
+    entry = load().kc_weighted_vote_groups_i8 if cells.dtype == torch.int8 else load().kc_weighted_vote_groups_i32
+    _bind(torch, cells)
+    check(entry(cells.data_ptr(), G, n, group_record.data_ptr(), cp, weight.data_ptr(), meta.data_ptr(), sums.data_ptr(),
+                _stream_ptr(torch, stream)))
+    return meta, sums
 
 
 def consensus_host(codes, none_code, vals, rel_eps=0.03, abs_eps=1e-6, device=0, out=None):
@@ -452,15 +496,39 @@ class PackedResult:
         self.close()
 
 
+def pack_logprobs(records_logprobs, pinned: bool = True):
+    """records_logprobs: per record, per candidate a sequence of token logprobs (record-major, like pack_texts' records) ->
+    (lp float32 array, lp_off int64 [R*n+1]): the packed form kc_consolidate_json_packed_weighted takes (lp in page-locked
+    memory when `pinned`)."""
+    import numpy as np
+    seqs = [s for rec in records_logprobs for s in rec]
+    lp_off = np.zeros(len(seqs) + 1, dtype=np.int64)
+    if seqs:
+        np.cumsum(np.fromiter((len(s) for s in seqs), dtype=np.int64, count=len(seqs)), out=lp_off[1:])
+    total = int(lp_off[-1])
+    lp = pinned_empty((max(total, 1),), np.float32) if pinned else np.empty(max(total, 1), dtype=np.float32)
+    if total:
+        lp[:total] = np.concatenate([np.asarray(s, dtype=np.float32) for s in seqs if len(s)])
+    return lp, lp_off
+
+
 def consolidate_json_packed(blob, off, n, rel_eps: float = 0.03, abs_eps: float = 1e-6, device: int = 0, threads: int = 0,
-                            flags: int = 0) -> PackedResult:
+                            flags: int = 0, logprobs=None) -> PackedResult:
     """H1g: the JSON-in / JSON-out consolidation with the JSON work on the device (kc_consolidate_json_packed).
-    blob uint8 array of all candidate texts, off int64 [R*n+1]; see pack_texts()."""
+    blob uint8 array of all candidate texts, off int64 [R*n+1]; see pack_texts().  logprobs = (lp, lp_off) from pack_logprobs():
+    the likelihood-weighted vote (kc_consolidate_json_packed_weighted; records it declines keep status 1)."""
     lib = load()
     R = (len(off) - 1) // n if n else 0
     h = ctypes.c_void_p()
-    check(lib.kc_consolidate_json_packed(blob.ctypes.data, off.ctypes.data, R, n, float(rel_eps), float(abs_eps), device, threads,
-                                         flags, ctypes.byref(h)))
+    if logprobs is None:
+        check(lib.kc_consolidate_json_packed(blob.ctypes.data, off.ctypes.data, R, n, float(rel_eps), float(abs_eps), device, threads,
+                                             flags, ctypes.byref(h)))
+    else:
+        import numpy as np
+        lp, lp_off = logprobs
+        assert lp.dtype == np.float32 and lp_off.dtype == np.int64 and len(lp_off) == len(off), "logprobs do not match the records"
+        check(lib.kc_consolidate_json_packed_weighted(blob.ctypes.data, off.ctypes.data, lp.ctypes.data, lp_off.ctypes.data, R, n,
+                                                      float(rel_eps), float(abs_eps), device, threads, flags, ctypes.byref(h)))
     return PackedResult(h, R)
 
 

@@ -14,6 +14,12 @@ parent_valid_frac products cu:1418,1433,1444) depends only on the input structur
 planning; the GPU fills in the leaves.  Multi-word string fields (the similarity medoid, cu:1221-1237) are recorded as
 medoid groups for K4 when every pair is a Levenshtein pair inside the kernel's contract (`Plan._medoid_on_device`);
 mixed payloads and the other similarity methods are computed by `k_llms_b200.utils.similarity` on the host.
+
+With `weighted=True` (ConsensusSettings.candidate_weighting == "likelihood", self-defined: DESIGN.md §5) every record comes with
+its candidates' token logprobs; each vote group also records the record and, per cell, the ORIGINAL candidate index of the value
+(consensus_dict / consensus_list keep only the candidates whose value is a dict / list, cu:1416,1431, so positions shift), and the
+vote groups are decided by K3 -> candidate weights -> kc_weighted_vote_groups_i32 instead of K1.  Numeric and medoid leaves are
+not weighted.
 """
 from __future__ import annotations
 
@@ -120,7 +126,7 @@ class Plan:
     """Leaf groups of one or many records, ready for one K1, one K2 and one K4 launch."""
 
     def __init__(self, n: int, allow_none_as_candidate: bool, rel_eps: float, abs_eps: float, host_primitive: Callable,
-                 numeric_branch: bool = True):
+                 numeric_branch: bool = True, weighted: bool = False):
         if n > MAX_CANDIDATES:
             raise ValueError(f"{n} candidates per request: k_llms_b200 consolidates at most {MAX_CANDIDATES} (one kernel row per "
                              "field holds every candidate; the package has no CPU path to fall back to)")
@@ -135,9 +141,14 @@ class Plan:
         self.num_rows: List[List[float]] = []
         self.medoid_groups: List[List[str]] = []  # normalised strings of the groups K4 handles
         self.string_method = "embeddings"         # set by the caller (ConsensusSettings.string_similarity_method)
+        self.weighted = weighted
+        self.rec_logprobs: List[Sequence[Sequence[float]]] = []  # weighted: per record, the token logprobs of each candidate
+        self.vote_rec: List[int] = []             # weighted: the record of each vote row
+        self.vote_cand: List[List[int]] = []      # weighted: the candidate of each cell of each vote row
+        self._rec = -1
 
     # -- leaves ---------------------------------------------------------------------------------------
-    def _vote(self, values: Sequence[Any], pvf: float) -> _VoteLeaf:
+    def _vote(self, values: Sequence[Any], pvf: float, cand: Sequence[int]) -> _VoteLeaf:
         first = next(v for v in values if v is not None)
         codes: List[int] = []
         table: dict = {}
@@ -155,6 +166,9 @@ class Plan:
                     codes.append(table.setdefault(k, len(table)))
         codes.extend([_native.CODE_ABSENT] * (self.n - len(codes)))
         self.vote_rows.append(codes)
+        if self.weighted:
+            self.vote_rec.append(self._rec)
+            self.vote_cand.append(list(cand) + [0] * (self.n - len(cand)))
         return _VoteLeaf(len(self.vote_rows) - 1, cells, pvf)
 
     def _numeric(self, values: Sequence[Any], pvf: float) -> _NumLeaf:
@@ -174,7 +188,17 @@ class Plan:
         return _NumLeaf(len(self.num_rows) - 1, list(values), pvf)
 
     # -- dispatcher (cu:1376-1454) ----------------------------------------------------------------------
-    def add(self, values: Sequence[Any], pvf: float, embed: Optional[Callable]):
+    def add(self, values: Sequence[Any], pvf: float, embed: Optional[Callable],
+            candidate_logprobs: Optional[Sequence[Sequence[float]]] = None):
+        """Plan one record; a weighted plan needs candidate_logprobs[c] = the token logprobs of values[c]."""
+        if self.weighted:
+            if candidate_logprobs is None or len(candidate_logprobs) != len(values):
+                raise ValueError("a likelihood-weighted plan needs the token logprobs of every candidate")
+            self.rec_logprobs.append(candidate_logprobs)
+            self._rec = len(self.rec_logprobs) - 1
+        return self._add(values, pvf, embed, range(len(values)))
+
+    def _add(self, values: Sequence[Any], pvf: float, embed: Optional[Callable], cand: Sequence[int]):
         if not values:
             return _Const(None, pvf)  # cu:1395-1396
         live = [v for v in values if v is not None]
@@ -182,9 +206,10 @@ class Plan:
             return _Const(None, 0.0)  # cu:1401-1402
         head = live[0]
         if isinstance(head, (str, bool)) and all(len(str(v).strip().split()) < 3 for v in live):
-            return self._vote(values, pvf)  # cu:1405-1411
+            return self._vote(values, pvf, cand)  # cu:1405-1411
         if isinstance(head, dict):  # cu:1414-1426 -> consensus_dict cu:1269-1306
-            dicts = [v for v in values if isinstance(v, dict)]
+            kept = [(c, v) for c, v in zip(cand, values) if isinstance(v, dict)]
+            dicts, sub_cand = [v for _, v in kept], [c for c, _ in kept]
             sub = pvf * (len(dicts) / len(values))
             keys: dict = {}
             for d in dicts:
@@ -194,13 +219,14 @@ class Plan:
             for k in keys:
                 if any(mark in k for mark in SKIPPED_KEY_MARKERS):
                     continue
-                children[k] = self.add([d.get(k) for d in dicts], sub, embed)
+                children[k] = self._add([d.get(k) for d in dicts], sub, embed, sub_cand)
             return _DictNode(children)
         if isinstance(head, list):  # cu:1429-1441 -> consensus_list cu:1309-1352
-            lists = [v for v in values if isinstance(v, list)]
+            kept = [(c, v) for c, v in zip(cand, values) if isinstance(v, list)]
+            lists, sub_cand = [v for _, v in kept], [c for c, _ in kept]
             sub = pvf * (len(lists) / len(values))
             longest = max(len(l) for l in lists)
-            return _ListNode([self.add([l[i] if i < len(l) else None for l in lists], sub, embed) for i in range(longest)])
+            return _ListNode([self._add([l[i] if i < len(l) else None for l in lists], sub, embed, sub_cand) for i in range(longest)])
         if embed is None:  # cu:1445-1446
             raise ValueError("sync_get_openai_embeddings_from_text is required for primitive consensus")
         try:
@@ -242,7 +268,14 @@ class Plan:
             raise RuntimeError("k_llms_b200: no CUDA device — the consensus hot path has no CPU fallback")
         dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         out = {}
-        if self.vote_rows:
+        if self.vote_rows and self.weighted:
+            codes = torch.from_numpy(np.asarray(self.vote_rows, dtype=np.int32)).to(dev)
+            meta, sums = _native.weighted_vote_groups(codes, torch.tensor(self.vote_rec, dtype=torch.int32, device=dev),
+                                                      self._candidate_weights(torch, dev),
+                                                      torch.from_numpy(np.asarray(self.vote_cand, dtype=np.int8)).to(dev))
+            out["vote_meta"] = meta.cpu().numpy().view(np.uint32)
+            out["vote_sums"] = sums.cpu().numpy()
+        elif self.vote_rows:
             codes = torch.from_numpy(np.asarray(self.vote_rows, dtype=np.int32)).to(dev)
             _, meta = _native.vote(codes, None)
             out["vote_meta"] = meta.cpu().numpy().view(np.uint32)
@@ -266,6 +299,22 @@ class Plan:
             out["medoid_idx"], out["medoid_avg"] = idx.cpu().numpy(), avg.cpu().numpy()
         return out
 
+    def _candidate_weights(self, torch, dev):
+        """K3 over every candidate's token logprobs, then the weight pre-pass: float32 [records, n].  A record with fewer than n
+        candidates fills the rest of its row with -3.0e38 (never the record's maximum, never referenced by a cell)."""
+        seqs = [s for rec in self.rec_logprobs for s in rec]
+        slots = [r * self.n + c for r, rec in enumerate(self.rec_logprobs) for c in range(len(rec))]
+        lens = np.fromiter((len(s) for s in seqs), dtype=np.int64, count=len(seqs))
+        offsets = np.zeros(len(seqs) + 1, dtype=np.int64)
+        np.cumsum(lens, out=offsets[1:])
+        flat = np.zeros(max(int(offsets[-1]), 1), dtype=np.float32)
+        if offsets[-1]:
+            flat[:offsets[-1]] = np.concatenate([np.asarray(s, dtype=np.float32) for s in seqs if len(s)])
+        sums = _native.logprob_sum(torch.from_numpy(flat).to(dev), torch.from_numpy(offsets).to(dev))
+        seq = torch.full((len(self.rec_logprobs) * self.n,), -3.0e38, dtype=torch.float32, device=dev)
+        seq[torch.tensor(slots, dtype=torch.int64, device=dev)] = sums
+        return _native.candidate_weights(seq.view(len(self.rec_logprobs), self.n))
+
     # -- epilogue --------------------------------------------------------------------------------------
     @staticmethod
     def _fields(m: int) -> Tuple[int, int, int, int, int]:
@@ -288,6 +337,9 @@ class Plan:
             idx, support, _nn, present, flags = self._fields(int(res["vote_meta"][node.row]))
             if not flags & _native.FLAG_HAS_VALUE:  # cannot happen for a planned vote group (>= 1 voter)
                 return None, (node.pvf if present == 0 else 0.0)
+            if "vote_sums" in res:  # likelihood-weighted: the weighted form of support / present (DESIGN.md §5)
+                w_win, w_present = res["vote_sums"][node.row]
+                return node.cells[idx], round(node.pvf * (float(w_win) / float(w_present)), 5)
             return node.cells[idx], round(node.pvf * (support / present), 5)  # cu:971,973,982
         idx, support, nn, present, flags = self._fields(int(res["num_meta"][node.row]))
         if flags & _native.FLAG_HAS_VALUE:

@@ -247,10 +247,11 @@ __global__ void __launch_bounds__(128) weighted_vote_kernel(const int32_t *__res
 }
 
 // The weighted vote of ONE group by one thread: rawrow = the group's cells (code >= 0, KC_CODE_NONE, absent < KC_CODE_NONE), nc = the
-// code None votes as (KC_CODE_NONE: it does not), w = the candidate weights of the group's record (shared memory).
+// code None votes as (KC_CODE_NONE: it does not), w = the weights of the group's cells (shared memory).  best_w = the winning class's
+// weight, total = the weight of the voting cells (both fp32 sums in cell order).
 template <int NP>
-__device__ __forceinline__ void weighted_core(const int32_t (&rawrow)[NP], int32_t nc, const float *w, int32_t &out_code,
-                                              uint32_t &out_meta, float &out_weight) {
+__device__ __forceinline__ void weighted_walk(const int32_t (&rawrow)[NP], int32_t nc, const float *w, int32_t &out_code,
+                                              uint32_t &out_meta, float &out_best_w, float &out_total) {
     using M = typename MaskOf<NP>::type;
     int32_t x[NP];
     M live = 0;
@@ -331,7 +332,16 @@ __device__ __forceinline__ void weighted_core(const int32_t (&rawrow)[NP], int32
     }
     out_code = best_code;
     out_meta = pack_meta(best_idx, best_cnt, voters, present, voters > 0 ? (KC_FLAG_HAS_VALUE | (tie ? KC_FLAG_TIE : 0u)) : 0u);
-    out_weight = voters > 0 ? __fdiv_rn(best_w, total) : 0.0f;
+    out_best_w = best_w;
+    out_total = total;
+}
+
+template <int NP>
+__device__ __forceinline__ void weighted_core(const int32_t (&rawrow)[NP], int32_t nc, const float *w, int32_t &out_code,
+                                              uint32_t &out_meta, float &out_weight) {
+    float best_w, total;
+    weighted_walk<NP>(rawrow, nc, w, out_code, out_meta, best_w, total);
+    out_weight = (KC_META_FLAGS(out_meta) & KC_FLAG_HAS_VALUE) ? __fdiv_rn(best_w, total) : 0.0f;
 }
 
 // K3b, weights once per record: the candidate weights depend on the record only, not on the field.  A CTA of T threads
@@ -703,24 +713,68 @@ __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS) weighted_vote_tma_kernel
 // ---- K3b with the weights OUT of the tile loop.  A pre-pass writes, once per record, the row [w_0 .. w_{N-1}, index of the heaviest
 // candidate, 3 pad words] (N + 4 floats: rows stay 16-byte multiples and consecutive rows start 4 banks apart); the vote kernel
 // fetches the rows of a tile's records with ONE cp.async.bulk next to the tile's tensor copy, completing on the same mbarrier.
+//
+// The same pre-pass gives the plain weight rows of kc_candidate_weights_f32: any n <= 64, row stride wrow = n (no pad words; with
+// wrow >= n + 4 the four pad words above follow the weights).  One warp per record, lane = candidate (and candidate + 32).
 
-template <int N>
-__global__ void __launch_bounds__(256) weight_rows_kernel(const float *__restrict__ seq_lp, int64_t n_records, float *__restrict__ rows) {
-    constexpr int WROW = N + 4;
+__global__ void __launch_bounds__(256) weight_rows_kernel(const float *__restrict__ seq_lp, int64_t n_records, int n, int wrow,
+                                                          float *__restrict__ rows) {
     const uint32_t lane = threadIdx.x & 31;
+    const bool lo_in = (int)lane < n, hi_in = (int)lane + 32 < n;
     const int64_t warp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     for (int64_t r = warp; r < n_records; r += n_warps) {
-        const float *s = seq_lp + r * N;
-        const float s_lo = __ldg(s + lane), s_hi = N > 32 ? __ldg(s + lane + 32) : -3.0e38f;
+        const float *s = seq_lp + r * n;
+        const float s_lo = lo_in ? __ldg(s + lane) : -3.0e38f, s_hi = hi_in ? __ldg(s + lane + 32) : -3.0e38f;
         float smax = fmaxf(s_lo, s_hi);
 #pragma unroll
         for (int st = 16; st >= 1; st >>= 1) smax = fmaxf(smax, __shfl_xor_sync(0xFFFFFFFFu, smax, st));
-        float *w = rows + r * WROW;
-        w[lane] = kexp(__fadd_rn(s_lo, -smax));
-        if (N > 32) w[lane + 32] = kexp(__fadd_rn(s_hi, -smax));
-        const uint32_t b_lo = __ballot_sync(0xFFFFFFFFu, s_lo == smax), b_hi = __ballot_sync(0xFFFFFFFFu, N > 32 && s_hi == smax);
-        const int imax = b_lo ? __ffs((int)b_lo) - 1 : (b_hi ? 31 + __ffs((int)b_hi) : N);
-        if (lane < 4) w[N + lane] = lane == 0 ? __int_as_float(imax) : 0.0f;
+        float *w = rows + r * wrow;
+        if (lo_in) w[lane] = kexp(__fadd_rn(s_lo, -smax));
+        if (hi_in) w[lane + 32] = kexp(__fadd_rn(s_hi, -smax));
+        if (wrow >= n + 4) {
+            const uint32_t b_lo = __ballot_sync(0xFFFFFFFFu, lo_in && s_lo == smax), b_hi = __ballot_sync(0xFFFFFFFFu, hi_in && s_hi == smax);
+            const int imax = b_lo ? __ffs((int)b_lo) - 1 : (b_hi ? 31 + __ffs((int)b_hi) : n);
+            if (lane < 4) w[n + lane] = lane == 0 ? __int_as_float(imax) : 0.0f;
+        }
+    }
+}
+
+// Likelihood-weighted vote over IRREGULAR groups (self-defined, DESIGN.md §5): group g belongs to record rec[g] and holds n cells
+// (K1's coding; CellT = int8 for the device JSON path's cell matrix, int32 for the planner's); cell i carries the weight of
+// candidate cand[g][i] (cand == NULL: candidate i) of its record.  The vote itself is K3b's (weighted_walk: class sums in cell
+// order, heaviest class, ties to the class seen first).  Out: K1's result word and (W_win, W_present), W_present = the fp32 sum of
+// the weights of the present cells (None cells included) in cell order.  One thread per group; its cells' weights sit in a
+// private shared-memory row (stride NP + 1: the rows of a warp's lanes start in different banks) for the walk to read.
+template <int NP, typename CellT>
+__global__ void __launch_bounds__(128) weighted_vote_groups_kernel(const CellT *__restrict__ cells, int64_t n_groups, int n,
+                                                                   const int32_t *__restrict__ rec, const int8_t *__restrict__ cand,
+                                                                   const float *__restrict__ weight, uint32_t *__restrict__ meta,
+                                                                   float2 *__restrict__ sums) {
+    __shared__ float wsh[128 * (NP + 1)];
+    float *w = wsh + threadIdx.x * (NP + 1);
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; g < n_groups; g += stride) {
+        const float *wr = weight + (int64_t)__ldg(rec + g) * n;
+        int32_t raw[NP];
+        float w_present = 0.0f;
+#pragma unroll
+        for (int i = 0; i < NP; ++i) {
+            const int32_t c = i < n ? (int32_t)__ldg(cells + g * n + i) : KC_CODE_ABSENT;
+            raw[i] = c;
+            float wi = 0.0f;
+            if (c >= KC_CODE_NONE) {
+                const int k = cand ? (int)__ldg(cand + g * n + i) : i;
+                wi = __ldg(wr + k);
+                w_present = __fadd_rn(w_present, wi);
+            }
+            w[i] = wi;
+        }
+        int32_t code;
+        uint32_t m;
+        float best_w, total;
+        weighted_walk<NP>(raw, KC_CODE_NONE, w, code, m, best_w, total);
+        meta[g] = m;
+        sums[g] = make_float2((KC_META_FLAGS(m) & KC_FLAG_HAS_VALUE) ? best_w : 0.0f, w_present);
     }
 }
 

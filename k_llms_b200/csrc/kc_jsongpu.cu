@@ -75,7 +75,8 @@ struct Worker {
     cudaStream_t stream = nullptr;
     cudaEvent_t ev[7] = {};
     DBuf text, off, fcount, slot, status, vbase, xbase, counters, toks, fdesc, piece_c, piece_l, vcells, xcells, win, vmeta, xvalue, xmeta,
-        len_c, len_l, out_c, out_l, scan_tmp, mcount, scount, ccount, mchars, mstr_off, mgrp_off, midx, mavg, nest, gpos;
+        len_c, len_l, out_c, out_l, scan_tmp, mcount, scount, ccount, mchars, mstr_off, mgrp_off, midx, mavg, nest, gpos,
+        lp, lp_off, seq_lp, cand_w, vrec, vsums;  // the last six: likelihood-weighted entry only
     PBuf h_small;  // totals and counters (pinned so the small D2H copies are asynchronous)
     PBuf h_scan;   // the scanned record offsets and the statuses of a chunk
     bool busy = false;
@@ -185,9 +186,14 @@ struct ChunkStage {  // per-chunk device-time split (CUDA events on the chunk's 
     float h2d = 0, plan = 0, kernels = 0, emit = 0, d2h = 0;
 };
 
-// One chunk on one worker: records [r0, r1) of the batch.
-int run_chunk(Worker &w, const char *h_text, const int64_t *h_off, int64_t r0, int64_t r1, int32_t n, double rel_eps, double abs_eps,
-              int sm_count, kc_json_result &res, ChunkStage &st) {
+__global__ void rebase_kernel(int64_t *off, int64_t count, int64_t base) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (int64_t)gridDim.x * blockDim.x) off[i] -= base;
+}
+
+// One chunk on one worker: records [r0, r1) of the batch.  h_lp / h_lp_off non-NULL: the likelihood-weighted vote (K3, the weight
+// pre-pass and kc_weighted_vote_groups_i8 in K1's place).
+int run_chunk(Worker &w, const char *h_text, const int64_t *h_off, const float *h_lp, const int64_t *h_lp_off, int64_t r0, int64_t r1,
+              int32_t n, double rel_eps, double abs_eps, int sm_count, kc_json_result &res, ChunkStage &st) {
     const int64_t Rc = r1 - r0;
     const int64_t b0 = h_off[r0 * n], b1 = h_off[r1 * n];
     const size_t bytes = (size_t)(b1 - b0);
@@ -242,6 +248,18 @@ int run_chunk(Worker &w, const char *h_text, const int64_t *h_off, int64_t r0, i
     KC_CUDA_I(cudaEventRecord(w.ev[0], s));
     KC_CUDA_I(cudaMemcpyAsync(w.text.p, h_text + b0, bytes, cudaMemcpyHostToDevice, s));
     KC_CUDA_I(cudaMemcpyAsync(w.off.p, h_off + r0 * n, (size_t)(Rc * n + 1) * 8, cudaMemcpyHostToDevice, s));
+    const bool weighted = h_lp_off != nullptr;
+    const int64_t l0 = weighted ? h_lp_off[r0 * n] : 0, n_tok = weighted ? h_lp_off[r1 * n] - l0 : 0;
+    if (weighted) {  // the chunk's token logprobs next to its texts, their offsets rebased to the chunk
+        R_(w.lp.reserve((size_t)std::max<int64_t>(n_tok, 4) * 4));
+        R_(w.lp_off.reserve((size_t)(Rc * n + 1) * 8));
+        R_(w.seq_lp.reserve((size_t)Rc * n * 4));
+        R_(w.cand_w.reserve((size_t)Rc * n * 4));
+        if (n_tok) KC_CUDA_I(cudaMemcpyAsync(w.lp.p, h_lp + l0, (size_t)n_tok * 4, cudaMemcpyHostToDevice, s));
+        KC_CUDA_I(cudaMemcpyAsync(w.lp_off.p, h_lp_off + r0 * n, (size_t)(Rc * n + 1) * 8, cudaMemcpyHostToDevice, s));
+        rebase_kernel<<<(int)std::min<int64_t>((Rc * n + 256) / 256, (int64_t)sm_count * 4), 256, 0, s>>>(w.lp_off.as<int64_t>(), Rc * n + 1, l0);
+        KC_CUDA_I(cudaGetLastError());
+    }
     KC_CUDA_I(cudaEventRecord(w.ev[1], s));
     nvtxRangePop();
     nvtxRangePushA("kc_json: plan (A0 count, A1 scan/type/encode)");
@@ -274,6 +292,11 @@ int run_chunk(Worker &w, const char *h_text, const int64_t *h_off, int64_t r0, i
     R_(w.vmeta.reserve(std::max<size_t>(T, 1) * 4));
     R_(w.xvalue.reserve(std::max<size_t>(T, 1) * 8));
     R_(w.xmeta.reserve(std::max<size_t>(T, 1) * 4));
+    if (weighted) {  // a record has at most one vote group per field slot
+        R_(w.vrec.reserve(std::max<size_t>(T, 1) * 4));
+        R_(w.vsums.reserve(std::max<size_t>(T, 1) * 8));
+        ch.vrec = w.vrec.as<int32_t>();
+    }
     ch.toks = w.toks.as<Tok>();
     ch.fdesc = w.fdesc.as<uint32_t>();
     ch.gpos = w.gpos.as<uint32_t>();
@@ -329,7 +352,14 @@ int run_chunk(Worker &w, const char *h_text, const int64_t *h_off, int64_t r0, i
     nvtxRangePop();
     nvtxRangePushA("kc_json: K1 vote + K2 numeric + K4 medoid");
     // K1 / K2 / K4: the same kernels as the columnar path (one "field" per group: local codes, no none_code table)
-    if (gv) R_(kc_vote_i8(ch.vcells, gv, n, nullptr, 1, w.win.as<int32_t>(), w.vmeta.as<uint32_t>(), s));
+    if (weighted) {  // K3 -> candidate weights -> the weighted vote (DESIGN.md §5); the logprob sums of the whole chunk are cheap
+        R_(kc_logprob_sum_f32(w.lp.as<float>(), w.lp_off.as<int64_t>(), Rc * n, w.seq_lp.as<float>(), s));
+        R_(kc_candidate_weights_f32(w.seq_lp.as<float>(), Rc, n, w.cand_w.as<float>(), s));
+        if (gv) R_(kc_weighted_vote_groups_i8(ch.vcells, gv, n, ch.vrec, nullptr, w.cand_w.as<float>(), w.vmeta.as<uint32_t>(), w.vsums.as<float>(), s));
+        ch.vsums = w.vsums.as<float>();
+    } else if (gv) {
+        R_(kc_vote_i8(ch.vcells, gv, n, nullptr, 1, w.win.as<int32_t>(), w.vmeta.as<uint32_t>(), s));
+    }
     if (gx) R_(kc_numeric_f64(ch.xcells, gx, n, rel_eps, abs_eps, w.xvalue.as<double>(), w.xmeta.as<uint32_t>(), s));
     if (gm) R_(kc_medoid_str(ch.mchars, ch.mstr_off, ch.mgrp_off, gm, std::max(2, n), w.midx.as<int32_t>(), w.mavg.as<double>(), s));
     KC_CUDA_I(cudaEventRecord(w.ev[3], s));
@@ -403,15 +433,26 @@ int run_chunk(Worker &w, const char *h_text, const int64_t *h_off, int64_t r0, i
 
 }  // namespace
 
-extern "C" {
+namespace {
 
-int kc_consolidate_json_packed(const char *h_text, const int64_t *h_off, int64_t n_records, int32_t n, double rel_eps, double abs_eps,
-                               int device, int32_t threads, uint32_t flags, kc_json_result **out) {
+// kc_consolidate_json_packed (h_lp_off == NULL) and kc_consolidate_json_packed_weighted: one implementation
+int consolidate_packed(const char *h_text, const int64_t *h_off, const float *h_lp, const int64_t *h_lp_off, int64_t n_records, int32_t n,
+                       double rel_eps, double abs_eps, int device, int32_t threads, uint32_t flags, kc_json_result **out) {
     if (!out) return kc_fail(KC_EINVAL, "kc_consolidate_json_packed: NULL out");
     *out = nullptr;
     if (n < 2 || n > KC_MAX_CANDIDATES) return kc_fail(KC_EINVAL, "kc_consolidate_json_packed: n=%d outside [2,%d]", n, KC_MAX_CANDIDATES);
     if (n_records < 0 || (n_records && (!h_text || !h_off))) return kc_fail(KC_EINVAL, "kc_consolidate_json_packed: bad arguments");
     if (!(rel_eps >= 0.0) || !(abs_eps >= 0.0)) return kc_fail(KC_EINVAL, "kc_consolidate_json_packed: rel_eps/abs_eps must be >= 0");
+    const bool weighted = h_lp_off != nullptr;
+    int64_t lp_bytes = 0;
+    if (weighted && n_records) {
+        if (h_lp_off[0] < 0) return kc_fail(KC_EINVAL, "kc_consolidate_json_packed_weighted: negative logprob offset");
+        for (int64_t i = 0; i < n_records * n; ++i)
+            if (h_lp_off[i + 1] < h_lp_off[i]) return kc_fail(KC_EINVAL, "kc_consolidate_json_packed_weighted: logprob offsets descend at %lld", (long long)i);
+        lp_bytes = (h_lp_off[n_records * n] - h_lp_off[0]) * 4;
+        if (lp_bytes && !h_lp) return kc_fail(KC_EINVAL, "kc_consolidate_json_packed_weighted: NULL logprobs");
+        flags |= KC_JSON_DEVICE_ONLY;  // the host path H1 does not weight: declined records are left to the caller
+    }
     const auto t_start = std::chrono::steady_clock::now();
     int prev = 0;
     KC_CUDA_I(cudaGetDevice(&prev));
@@ -450,11 +491,14 @@ int kc_consolidate_json_packed(const char *h_text, const int64_t *h_off, int64_t
         int64_t r = 0;
         while (r < R) {
             // records are a few KB: advance by estimate, then adjust
-            const int64_t start = h_off[r * n];
+            // the chunk's bytes: its texts, and with weighting its token logprobs
+            auto span = [&](int64_t a, int64_t b) -> size_t {
+                return (size_t)(h_off[b * n] - h_off[a * n]) + (weighted ? (size_t)(h_lp_off[b * n] - h_lp_off[a * n]) * 4 : 0);
+            };
             int64_t lo = r + 1, hi = R;
             while (lo < hi) {  // largest r1 with bytes(r, r1) <= chunk_bytes (at least one record)
                 const int64_t mid = lo + (hi - lo + 1) / 2;
-                if ((size_t)(h_off[mid * n] - start) <= chunk_bytes) lo = mid;
+                if (span(r, mid) <= chunk_bytes) lo = mid;
                 else hi = mid - 1;
             }
             r = lo;
@@ -478,7 +522,8 @@ int kc_consolidate_json_packed(const char *h_text, const int64_t *h_off, int64_t
         while (!rc) {
             const int k = next.fetch_add(1);
             if (k >= n_chunks) break;
-            rc = run_chunk(w, h_text, h_off, cuts[(size_t)k], cuts[(size_t)k + 1], n, rel_eps, abs_eps, sm_count, *res, stages[(size_t)wi]);
+            rc = run_chunk(w, h_text, h_off, h_lp, h_lp_off, cuts[(size_t)k], cuts[(size_t)k + 1], n, rel_eps, abs_eps, sm_count, *res,
+                           stages[(size_t)wi]);
         }
         if (rc) {
             cudaStreamSynchronize(w.stream);
@@ -563,7 +608,7 @@ int kc_consolidate_json_packed(const char *h_text, const int64_t *h_off, int64_t
     s.n_device = R - n_declined;
     s.n_host = n_host;
     s.n_python = n_declined - n_host;
-    s.input_bytes = total_bytes;
+    s.input_bytes = total_bytes + lp_bytes;
     s.output_bytes = res->used.load();
     s.chunks = n_chunks;
     s.streams = n_workers;
@@ -579,6 +624,22 @@ int kc_consolidate_json_packed(const char *h_text, const int64_t *h_off, int64_t
     s.wall_ms = ms(t_start, t_end);
     *out = res;
     return KC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int kc_consolidate_json_packed(const char *h_text, const int64_t *h_off, int64_t n_records, int32_t n, double rel_eps, double abs_eps,
+                               int device, int32_t threads, uint32_t flags, kc_json_result **out) {
+    return consolidate_packed(h_text, h_off, nullptr, nullptr, n_records, n, rel_eps, abs_eps, device, threads, flags, out);
+}
+
+int kc_consolidate_json_packed_weighted(const char *h_text, const int64_t *h_off, const float *h_lp, const int64_t *h_lp_off,
+                                        int64_t n_records, int32_t n, double rel_eps, double abs_eps, int device, int32_t threads,
+                                        uint32_t flags, kc_json_result **out) {
+    if (n_records > 0 && !h_lp_off) return kc_fail(KC_EINVAL, "kc_consolidate_json_packed_weighted: NULL logprob offsets");
+    return consolidate_packed(h_text, h_off, h_lp, h_lp_off, n_records, n, rel_eps, abs_eps, device, threads, flags, out);
 }
 
 int kc_json_result_view(kc_json_result *res, const char **text, const int64_t **content_off, const int64_t **content_len,
@@ -617,6 +678,7 @@ struct kc_debug_jsongpu {
     std::vector<uint8_t> mchars;
     std::vector<int32_t> mstr_off, mgrp_off;
     std::vector<int8_t> vcells;
+    std::vector<int32_t> vrec;
     std::vector<double> xcells;
     std::vector<int64_t> len_c, len_l;
     std::vector<uint8_t> out_c, out_l;
@@ -669,6 +731,8 @@ int kc_debug_jsongpu_plan(const char *h_text, const int64_t *h_off, int64_t n_re
     h->piece_l.assign(std::max<size_t>(T, 1), 0);
     h->vcells.assign(std::max<size_t>(T * n, 16), (int8_t)-1);
     h->xcells.assign(std::max<size_t>(T * n, 2), 0.0);
+    h->vrec.assign(std::max<size_t>(T, 1), 0);
+    ch.vrec = h->vrec.data();  // written by slots_phase; only the weighted emit reads what it says
     ch.toks = h->toks.data();
     ch.fdesc = h->fdesc.data();
     ch.gpos = h->gpos.data();
@@ -765,6 +829,24 @@ int kc_debug_jsongpu_emit(kc_debug_jsongpu *h, const uint32_t *vote_meta, const 
     if (likelihoods) *likelihoods = (const char *)h->out_l.data();
     if (likelihoods_off) *likelihoods_off = h->len_l.data();
     return KC_OK;
+}
+
+// the record of every vote group (what kc_weighted_vote_groups_i8 takes as d_group_record)
+int kc_debug_jsongpu_vote_records(const kc_debug_jsongpu *h, const int32_t **vote_records) {
+    if (!h || !vote_records) return KC_EINVAL;
+    *vote_records = h->vrec.data();
+    return KC_OK;
+}
+
+// kc_debug_jsongpu_emit with the weighted vote's (W_win, W_present) per vote group: the confidences of the weighted entry
+int kc_debug_jsongpu_emit_weighted(kc_debug_jsongpu *h, const uint32_t *vote_meta, const float *vote_sums, const double *num_value,
+                                   const uint32_t *num_meta, const char **content, const int64_t **content_off, const char **likelihoods,
+                                   const int64_t **likelihoods_off) {
+    if (!h || !vote_sums) return KC_EINVAL;
+    h->ch.vsums = vote_sums;
+    const int rc = kc_debug_jsongpu_emit(h, vote_meta, num_value, num_meta, content, content_off, likelihoods, likelihoods_off);
+    h->ch.vsums = nullptr;
+    return rc;
 }
 
 void kc_debug_jsongpu_free(kc_debug_jsongpu *h) { delete h; }

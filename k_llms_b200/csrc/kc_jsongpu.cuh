@@ -68,6 +68,8 @@ struct Chunk {
     const int32_t *midx;                 // K4 results: medoid's index within its group,
     const double *mavg;                  //             its mean similarity
     const uint32_t *vmeta;   // K1 result words
+    int32_t *vrec;           // likelihood-weighted entry only (else NULL): [vote groups] the record of each vote group (slots)
+    const float *vsums;      // likelihood-weighted entry only (else NULL): [vote groups][2] (W_win, W_present) of the weighted vote
     const double *xvalue;    // K2 values
     const uint32_t *xmeta;   // K2 result words
     uint32_t *piece_c, *piece_l;  // [slots] by (slot + rank): piece length, then (after the leader's pass) piece offset
@@ -317,6 +319,8 @@ KC_HD inline void slots_phase(const Chunk &ch, int32_t r) {
     ch.counters[1] += nx;
     ch.counters[2] += nm;
 #endif
+    if (ch.vrec)  // the weighted vote finds the record's weight row through it; a record's groups are contiguous
+        for (uint32_t k = 0; k < nv; ++k) ch.vrec[ch.vbase[r] + k] = r;
 }
 
 // A2, after the exclusive scans of mcount / scount / ccount: lane j writes its medoid group in K4's CSR form.  Group, string
@@ -415,7 +419,12 @@ KC_HD inline void format_field(const Chunk &ch, int32_t r, int32_t j, Sink &cont
         } else {
             content.json_string(ch.text + row[idx].vstart, row[idx].vlen, row[idx].flags & TOK_ESCAPED);  // first original whose sanitised form wins (cu:971)
         }
-        conf = py_round5(1.0 * ((double)support / (double)present));
+        if (ch.vsums) {  // likelihood-weighted: the weighted form of support / present (DESIGN.md §5)
+            const float *ws = ch.vsums + 2 * ((int64_t)ch.vbase[r] + g);
+            conf = py_round5(1.0 * ((double)ws[0] / (double)ws[1]));
+        } else {
+            conf = py_round5(1.0 * ((double)support / (double)present));
+        }
     } else if (kind == F_NUMERIC) {
         const uint32_t m = ch.xmeta[(int64_t)ch.xbase[r] + g];
         const uint32_t idx = KC_META_IDX(m), support = KC_META_SUPPORT(m), nn = KC_META_NN(m), present = KC_META_PRESENT(m);

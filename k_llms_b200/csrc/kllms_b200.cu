@@ -799,7 +799,7 @@ int kc_weighted_vote_i32(const int32_t *d_codes, const float *d_seq_logprob, int
                 float *d_rows = nullptr;
                 KC_CUDA(cudaMallocAsync(reinterpret_cast<void **>(&d_rows), (size_t)n_records * WROW * 4, st));
                 const int pre_grid = (int)std::min<int64_t>((n_records + 7) / 8, (int64_t)info.sm_count * 8);
-                pre_kernel<<<pre_grid, 256, 0, st>>>(d_seq_logprob, n_records, d_rows);
+                pre_kernel<<<pre_grid, 256, 0, st>>>(d_seq_logprob, n_records, N, WROW, d_rows);
                 int rc2 = cudaGetLastError() == cudaSuccess ? KC_OK : fail(KC_ECUDA, "kc_weighted_vote_i32: weight_rows_kernel launch failed");
                 const size_t smem = (size_t)WARPS * STAGES * 32 * N * 4 + 1024 + (size_t)WARPS * (STAGES + 1) * rec_cap0 * WROW * 4;
                 const int64_t slab = std::max<int64_t>(n_fields, kMaxGroupsPerLaunch / n_fields * n_fields);
@@ -818,7 +818,7 @@ int kc_weighted_vote_i32(const int32_t *d_codes, const float *d_seq_logprob, int
                 cudaFreeAsync(d_rows, st);
                 return rc2;
             };
-            return launch_rows(kc::weight_rows_kernel<32>, kc::weighted_vote_rows_kernel<32, 8, 2, 3>, 32, 8, 2);
+            return launch_rows(kc::weight_rows_kernel, kc::weighted_vote_rows_kernel<32, 8, 2, 3>, 32, 8, 2);
         }
         // measured on B200 (profiles/r2_k3b_variants.txt): n = 32 with 3 CTAs / SM (80 registers) and the logprobs requested a tile ahead;
         // n = 64 (2 x the registers per row) without the prefetch
@@ -852,6 +852,63 @@ int kc_weighted_vote_i32(const int32_t *d_codes, const float *d_seq_logprob, int
 #undef KC_WV
     KC_CUDA(cudaGetLastError());
     return KC_OK;
+}
+
+int kc_candidate_weights_f32(const float *d_seq_logprob, int64_t n_records, int32_t n, float *d_weight, void *stream) {
+    if (n < 1 || n > KC_MAX_CANDIDATES) return fail(KC_EINVAL, "kc_candidate_weights_f32: n=%d outside [1,%d]", n, KC_MAX_CANDIDATES);
+    if (n_records < 0) return fail(KC_EINVAL, "kc_candidate_weights_f32: negative n_records");
+    if (n_records == 0) return KC_OK;
+    if (!d_seq_logprob || !d_weight) return fail(KC_EINVAL, "kc_candidate_weights_f32: NULL buffer");
+    DeviceInfo info;
+    int rc = device_info(info);
+    if (rc) return rc;
+    const int grid = (int)std::min<int64_t>((n_records + 7) / 8, (int64_t)info.sm_count * 8);
+    kc::weight_rows_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(d_seq_logprob, n_records, n, n, d_weight);
+    KC_CUDA(cudaGetLastError());
+    return KC_OK;
+}
+
+static int weighted_vote_groups(const char *what, const void *d_cells, bool i8, int64_t n_groups, int32_t n, const int32_t *d_group_record,
+                                const int8_t *d_cand, const float *d_weight, uint32_t *d_meta, float *d_sums, void *stream) {
+    if (n < 1 || n > KC_MAX_CANDIDATES) return fail(KC_EINVAL, "%s: n=%d outside [1,%d]", what, n, KC_MAX_CANDIDATES);
+    if (n_groups < 0) return fail(KC_EINVAL, "%s: negative n_groups", what);
+    if (n_groups == 0) return KC_OK;
+    if (!d_cells || !d_group_record || !d_weight || !d_meta || !d_sums) return fail(KC_EINVAL, "%s: NULL buffer", what);
+    if (((uintptr_t)d_sums) & 7) return fail(KC_EINVAL, "%s: d_sums must be 8-byte aligned", what);
+    DeviceInfo info;
+    int rc = device_info(info);
+    if (rc) return rc;
+    const int threads = 128;
+    const int grid = (int)std::min<int64_t>((n_groups + threads - 1) / threads, (int64_t)info.sm_count * 8);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    float2 *sums = reinterpret_cast<float2 *>(d_sums);
+#define KC_WVG(NP)                                                                                                                              \
+    do {                                                                                                                                    \
+        if (i8)                                                                                                                             \
+            kc::weighted_vote_groups_kernel<NP, int8_t><<<grid, threads, 0, st>>>(static_cast<const int8_t *>(d_cells), n_groups, n,     \
+                                                                                  d_group_record, d_cand, d_weight, d_meta, sums);      \
+        else                                                                                                                                \
+            kc::weighted_vote_groups_kernel<NP, int32_t><<<grid, threads, 0, st>>>(static_cast<const int32_t *>(d_cells), n_groups, n,   \
+                                                                                   d_group_record, d_cand, d_weight, d_meta, sums);     \
+    } while (0)
+    if (n <= 16) KC_WVG(16);  // (an 8-cell instance of the int8 kernel spills 16 bytes: the 16-cell one does not)
+    else if (n <= 32) KC_WVG(32);
+    else KC_WVG(64);
+#undef KC_WVG
+    KC_CUDA(cudaGetLastError());
+    return KC_OK;
+}
+
+int kc_weighted_vote_groups_i8(const int8_t *d_cells, int64_t n_groups, int32_t n, const int32_t *d_group_record, const int8_t *d_cand,
+                               const float *d_weight, uint32_t *d_meta, float *d_sums, void *stream) {
+    return weighted_vote_groups("kc_weighted_vote_groups_i8", d_cells, true, n_groups, n, d_group_record, d_cand, d_weight, d_meta, d_sums,
+                                stream);
+}
+
+int kc_weighted_vote_groups_i32(const int32_t *d_cells, int64_t n_groups, int32_t n, const int32_t *d_group_record, const int8_t *d_cand,
+                                const float *d_weight, uint32_t *d_meta, float *d_sums, void *stream) {
+    return weighted_vote_groups("kc_weighted_vote_groups_i32", d_cells, false, n_groups, n, d_group_record, d_cand, d_weight, d_meta, d_sums,
+                                stream);
 }
 
 int kc_medoid_str(const uint8_t *d_chars, const int32_t *d_str_off, const int32_t *d_grp_off, int64_t n_groups,

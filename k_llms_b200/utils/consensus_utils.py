@@ -13,6 +13,7 @@ from __future__ import annotations
 
 import asyncio
 import logging
+import math
 import warnings
 from typing import Any, Awaitable, Callable, List, Literal, Optional, Sequence, Tuple
 
@@ -25,6 +26,7 @@ logger = logging.getLogger(__name__)
 
 StringSimilarityMethod = Literal["levenshtein", "jaccard", "hamming", "embeddings"]
 StringConsensusMethod = Literal["centroid", "llm-consensus"]
+CandidateWeighting = Literal["uniform", "likelihood"]
 SYNC_GET_OPENAI_EMBEDDINGS_FROM_TEXT_TYPE = Callable[[List[str]], List[List[float]]]
 ASYNC_GET_OPENAI_EMBEDDINGS_FROM_TEXT_TYPE = Callable[[List[str]], Awaitable[List[List[float]]]]
 
@@ -32,7 +34,11 @@ ASYNC_GET_OPENAI_EMBEDDINGS_FROM_TEXT_TYPE = Callable[[List[str]], Awaitable[Lis
 class ConsensusSettings(BaseModel):
     """Same fields and defaults as the reference model (cu:53-69).  Only allow_none_as_candidate,
     string_similarity_method, string_consensus_method, min_support_ratio, rel_eps and abs_eps are read by
-    the reference's code paths; the others are accepted for compatibility."""
+    the reference's code paths; the others are accepted for compatibility.
+
+    candidate_weighting is this package's own (self-defined, DESIGN.md §5): "uniform" (default) is the reference's vote;
+    "likelihood" weights every candidate's vote in str/bool fields by exp(s_c - max_k s_k), s_c = the sum of the candidate's
+    token logprobs.  Numeric fields, similarity-medoid fields and the list alignment are not weighted."""
 
     allow_none_as_candidate: bool = False
     string_similarity_method: StringSimilarityMethod = "embeddings"
@@ -44,6 +50,28 @@ class ConsensusSettings(BaseModel):
     base_maj_thresh: float = 0.6
     maj_loosen_k: float = 0.1
     trim_frac: float = 0.2
+    candidate_weighting: CandidateWeighting = "uniform"
+
+
+def check_candidate_logprobs(settings: ConsensusSettings, candidate_logprobs, n: int):
+    """The logprobs a likelihood-weighted consolidation runs on: candidate_logprobs[c] = the token logprobs of candidate c (one
+    sequence per candidate), as lists of floats; None under uniform weighting.  Raises ValueError when they are missing, do not
+    match the n candidates, or hold a NaN."""
+    if settings.candidate_weighting != "likelihood":
+        return None
+    if candidate_logprobs is None:
+        raise ValueError("candidate_weighting='likelihood' needs the token logprobs of every candidate (request logprobs=True)")
+    if len(candidate_logprobs) != n:
+        raise ValueError(f"candidate_weighting='likelihood': {len(candidate_logprobs)} logprob sequences for {n} candidates")
+    out = []
+    for c, seq in enumerate(candidate_logprobs):
+        if seq is None:
+            raise ValueError(f"candidate_weighting='likelihood': candidate {c} has no logprobs (request logprobs=True)")
+        seq = [float(x) for x in seq]
+        if any(math.isnan(x) for x in seq):
+            raise ValueError(f"candidate_weighting='likelihood': candidate {c} has a NaN logprob")
+        out.append(seq)
+    return out
 
 
 def _host_primitive(settings: ConsensusSettings):
@@ -58,7 +86,7 @@ def _host_primitive(settings: ConsensusSettings):
 
 def _plan_for(n: int, settings: ConsensusSettings, numeric_branch: bool = True) -> columnar.Plan:
     plan = columnar.Plan(n, settings.allow_none_as_candidate, settings.rel_eps, settings.abs_eps, _host_primitive(settings),
-                         numeric_branch=numeric_branch)
+                         numeric_branch=numeric_branch, weighted=settings.candidate_weighting == "likelihood")
     plan.string_method = settings.string_similarity_method if settings.string_consensus_method == "centroid" else "host"
     return plan
 
@@ -70,10 +98,14 @@ def consensus_values(
     client: Any,
     parent_valid_frac: float = 1.0,
     _numeric_branch: bool = True,
+    *,
+    candidate_logprobs: Optional[Sequence[Sequence[float]]] = None,
 ) -> Tuple[Any, Any]:
-    """(consensus value, confidence) for one record's n candidate values — cu:1376-1454."""
+    """(consensus value, confidence) for one record's n candidate values — cu:1376-1454.  With
+    consensus_settings.candidate_weighting == "likelihood", candidate_logprobs[c] = the token logprobs of values[c]."""
+    lps = check_candidate_logprobs(consensus_settings, candidate_logprobs, len(values))
     plan = _plan_for(len(values), consensus_settings, _numeric_branch)
-    root = plan.add(values, parent_valid_frac, sync_get_openai_embeddings_from_text)
+    root = plan.add(values, parent_valid_frac, sync_get_openai_embeddings_from_text, lps)
     res = plan.run() if (plan.vote_rows or plan.num_rows or plan.medoid_groups) else {}
     return plan.materialise(root, res)
 
@@ -84,12 +116,19 @@ def consensus_values_batch(
     sync_get_openai_embeddings_from_text: Optional[SYNC_GET_OPENAI_EMBEDDINGS_FROM_TEXT_TYPE] = None,
     client: Any = None,
     parent_valid_frac: float = 1.0,
+    *,
+    candidate_logprobs: Optional[Sequence[Sequence[Sequence[float]]]] = None,
 ) -> List[Tuple[Any, Any]]:
-    """Batched entry (new): consensus_values for many independent records with ONE K1 and ONE K2 launch."""
+    """Batched entry (new): consensus_values for many independent records with ONE K1 and ONE K2 launch.  With likelihood
+    weighting, candidate_logprobs[r][c] = the token logprobs of records[r][c]."""
     settings = consensus_settings or ConsensusSettings()
     embed = sync_get_openai_embeddings_from_text if sync_get_openai_embeddings_from_text is not None else _no_embeddings
+    if settings.candidate_weighting == "likelihood" and (candidate_logprobs is None or len(candidate_logprobs) != len(records)):
+        raise ValueError("candidate_weighting='likelihood' needs one list of candidate logprobs per record")
+    lps = [check_candidate_logprobs(settings, candidate_logprobs[i] if candidate_logprobs is not None else None, len(values))
+           for i, values in enumerate(records)]
     plan = _plan_for(max((len(r) for r in records), default=1), settings)
-    roots = [plan.add(values, parent_valid_frac, embed) for values in records]
+    roots = [plan.add(values, parent_valid_frac, embed, lp) for values, lp in zip(records, lps)]
     res = plan.run() if (plan.vote_rows or plan.num_rows or plan.medoid_groups) else {}
     return [plan.materialise(root, res) for root in roots]
 
@@ -104,6 +143,8 @@ async def async_consensus_values(
     async_get_openai_embeddings_from_text: ASYNC_GET_OPENAI_EMBEDDINGS_FROM_TEXT_TYPE,
     client: Any,
     parent_valid_frac: float = 1.0,
+    *,
+    candidate_logprobs: Optional[Sequence[Sequence[float]]] = None,
 ) -> Tuple[Any, Any]:
     """Async twin (cu:1779-1860).  The reference's async primitive has NO numeric clustering (cu:1638-1688, SURVEY.md §0.5):
     a non-unanimous numeric field takes the similarity medoid — [10, 10, 11] gives (10, 0.5) here and (10.0, 0.66667) in the
@@ -117,7 +158,7 @@ async def async_consensus_values(
 
     return await asyncio.to_thread(consensus_values, values, consensus_settings,
                                    embed if async_get_openai_embeddings_from_text is not None else None, client,
-                                   parent_valid_frac, False)
+                                   parent_valid_frac, False, candidate_logprobs=candidate_logprobs)
 
 
 # ----------------------------------------------------------------------------- alignment pre-pass

@@ -23,6 +23,7 @@ from .consensus_utils import (
     ConsensusSettings,
     async_consensus_values,
     async_recursive_list_alignments,
+    check_candidate_logprobs,
     consensus_values,
     recursive_list_alignments,
 )
@@ -49,6 +50,17 @@ def _contents_of(choices) -> List[dict]:
     return [_safe_parse_content(c.message.content) for c in choices if c.message.content]
 
 
+def _logprobs_of(choices, settings) -> Optional[List[List[float]]]:
+    """Under likelihood weighting, the token logprobs (choice.logprobs.content[*].logprob) of the choices _contents_of keeps: a
+    dropped choice's logprobs are dropped with it.  None under uniform weighting."""
+    if settings.candidate_weighting != "likelihood":
+        return None
+    kept = [c for c in choices if c.message.content]
+    seqs = [[t.logprob for t in c.logprobs.content] if c.logprobs is not None and c.logprobs.content is not None else None
+            for c in kept]
+    return check_candidate_logprobs(settings, seqs, len(kept))
+
+
 def _native_alignment(contents, settings):
     """The alignment pre-pass in native code (H2, `kc_align_json`: same result as `recursive_list_alignments`, pinned on the
     reference's goldens) — or None when the record needs the Python pre-pass: another similarity method than the default,
@@ -65,7 +77,7 @@ def _native_settings(settings) -> bool:
             and settings.string_consensus_method == "centroid" and settings.min_support_ratio == 0.51)
 
 
-def _consensus_of_choices_native(choices, settings, embed):
+def _consensus_of_choices_native(choices, settings, embed, logprobs=None):
     """The whole per-request path in native code (H1): the n `choice.message.content` texts in -> (consensus value,
     likelihoods), i.e. parse + alignment pre-pass + vote / numeric / medoid kernels + decode — or None when the request needs
     the Python path (non-default settings, fewer than two non-empty contents, anything H1 declines; no embeddings callable:
@@ -76,7 +88,7 @@ def _consensus_of_choices_native(choices, settings, embed):
     texts = [c.message.content for c in choices if c.message.content]  # the filter of _contents_of (reference consolidation.py:92)
     if len(texts) < 2 or len(texts) > _native.MAX_CANDIDATES or not _native_settings(settings):
         return None
-    out = _combiner.run(texts, settings.rel_eps, settings.abs_eps)
+    out = _combiner.run(texts, settings.rel_eps, settings.abs_eps, logprobs)
     if out is None:
         return None
     content_text, likelihoods_text = out
@@ -89,13 +101,23 @@ def _consensus_of_choices_native(choices, settings, embed):
     return value, json.loads(likelihoods_text)
 
 
-def _native_consolidate(records, rel_eps, abs_eps, device: int = 0):
+def _native_consolidate(records, rel_eps, abs_eps, device: int = 0, logprobs=None):
     """records of n candidate texts -> [(content, likelihoods text) or None]: the device JSON path (H1g,
     kc_consolidate_json_packed: scan / key sort / typing / encode / K1 + K2 / emit on the GPU; re-entrant, pooled streams), which
-    hands what it does not model to the host path (H1, kc_consolidate_json) inside the same call."""
+    hands what it does not model to the host path (H1, kc_consolidate_json) inside the same call.  logprobs[r][c] = the token
+    logprobs of records[r][c]: the likelihood-weighted entry (kc_consolidate_json_packed_weighted), which has no host path — what
+    the device declines comes back as None."""
+    import numpy as np
+
     from .. import _native
-    blob, off, n = _native.pack_texts(records, pinned=len(records) >= 256)  # page-locking only pays for batches
-    res = _native.consolidate_json_packed(blob, off, n, rel_eps, abs_eps, device)
+    pinned = len(records) >= 256  # page-locking only pays for batches
+    blob, off, n = _native.pack_texts(records, pinned=pinned)
+    lp = None
+    if logprobs is not None:
+        lp = _native.pack_logprobs(logprobs, pinned=pinned)
+        if np.isnan(lp[0][:lp[1][-1]]).any():
+            raise ValueError("candidate_weighting='likelihood': a candidate has a NaN logprob")
+    res = _native.consolidate_json_packed(blob, off, n, rel_eps, abs_eps, device, logprobs=lp)
     try:
         return res.pairs()
     finally:
@@ -122,11 +144,12 @@ class _Combiner:
             if not batch:
                 return
             groups: dict = {}
-            for item in batch:
-                groups.setdefault((len(item["texts"]), item["eps"]), []).append(item)
-            for (_n, eps), items in groups.items():
+            for item in batch:  # one call per candidate count, eps and weighting
+                groups.setdefault((len(item["texts"]), item["eps"], item["lp"] is not None), []).append(item)
+            for (_n, eps, weighted), items in groups.items():
                 try:
-                    outs = _native_consolidate([it["texts"] for it in items], eps[0], eps[1])
+                    outs = _native_consolidate([it["texts"] for it in items], eps[0], eps[1],
+                                               logprobs=[it["lp"] for it in items] if weighted else None)
                     for it, o in zip(items, outs):
                         it["out"] = o
                 except BaseException as exc:  # hand the failure to every waiter of the group
@@ -135,9 +158,9 @@ class _Combiner:
                 for it in items:
                     it["done"].set()
 
-    def run(self, texts, rel_eps, abs_eps):
+    def run(self, texts, rel_eps, abs_eps, logprobs=None):
         import threading
-        item = {"texts": texts, "eps": (rel_eps, abs_eps), "done": threading.Event(), "out": None, "err": None}
+        item = {"texts": texts, "eps": (rel_eps, abs_eps), "lp": logprobs, "done": threading.Event(), "out": None, "err": None}
         with self._qlock:
             self._queue.append(item)
         while not item["done"].is_set():
@@ -163,23 +186,23 @@ def _check_candidates(n: int) -> None:
                          "(README.md, Limits)")
 
 
-def _consensus_sync(contents, settings, embed, client):
+def _consensus_sync(contents, settings, embed, client, logprobs=None):
     if len(contents) >= 2:  # reference consolidation.py:96-104
         aligned = _native_alignment(contents, settings)
         if aligned is None:
             aligned, _ = recursive_list_alignments(contents, settings.string_similarity_method, embed, client, settings.min_support_ratio)
         contents = [(d if isinstance(d, dict) else {}) for d in aligned]
-    return consensus_values(contents, settings, embed, client=client)
+    return consensus_values(contents, settings, embed, client=client, candidate_logprobs=logprobs)
 
 
-async def _consensus_async(contents, settings, embed, client):
+async def _consensus_async(contents, settings, embed, client, logprobs=None):
     if len(contents) >= 2:
         aligned = _native_alignment(contents, settings)
         if aligned is None:
             aligned, _ = await async_recursive_list_alignments(contents, settings.string_similarity_method, embed, client,
                                                                settings.min_support_ratio)
         contents = [(d if isinstance(d, dict) else {}) for d in aligned]
-    return await async_consensus_values(contents, settings, embed, client=client)
+    return await async_consensus_values(contents, settings, embed, client=client, candidate_logprobs=logprobs)
 
 
 def _assemble_plain(base: ChatCompletion, heads, consensus_content, likelihoods) -> KLLMsChatCompletion:
@@ -214,8 +237,10 @@ def consolidate_chat_completions(
         if len(completion.choices) == 1:
             return KLLMsChatCompletion.model_validate(completion.model_dump())
         _check_candidates(len(completion.choices))
-        content, likelihoods = (_consensus_of_choices_native(completion.choices, consensus_settings, get_openai_embeddings_from_text)
-                                or _consensus_sync(_contents_of(completion.choices), consensus_settings, get_openai_embeddings_from_text, client))
+        lps = _logprobs_of(completion.choices, consensus_settings)
+        content, likelihoods = (_consensus_of_choices_native(completion.choices, consensus_settings, get_openai_embeddings_from_text, lps)
+                                or _consensus_sync(_contents_of(completion.choices), consensus_settings, get_openai_embeddings_from_text, client,
+                                                   lps))
         return _assemble_plain(completion, list(completion.choices), content, likelihoods)
     completion_list = completions
     assert len(completion_list) > 0, "Cannot consolidate empty list of completions"
@@ -226,8 +251,9 @@ def consolidate_chat_completions(
     # 176-216); a completion without choices contributes nothing
     firsts = [(i, c.choices[0]) for i, c in enumerate(completion_list) if c.choices]
     heads = [c for _, c in firsts]
-    content, likelihoods = (_consensus_of_choices_native(heads, consensus_settings, get_openai_embeddings_from_text)
-                            or _consensus_sync(_contents_of(heads), consensus_settings, get_openai_embeddings_from_text, client))
+    lps = _logprobs_of(heads, consensus_settings)
+    content, likelihoods = (_consensus_of_choices_native(heads, consensus_settings, get_openai_embeddings_from_text, lps)
+                            or _consensus_sync(_contents_of(heads), consensus_settings, get_openai_embeddings_from_text, client, lps))
     out = _assemble_plain(completion_list[0], heads, content, likelihoods)
     for k, (i, _) in enumerate(firsts):
         out.choices[k + 1].index = i + 1
@@ -248,7 +274,8 @@ async def async_consolidate_chat_completions(
     # the native JSON paths implement the SYNC semantics; the reference's async dispatcher differs on numeric fields
     # (cu:1638-1688: no clustering), so the async entry points plan in Python (async_consensus_values) — votes still on the GPU
     content, likelihoods = await _consensus_async(_contents_of(completion.choices), consensus_settings,
-                                                  async_get_openai_embeddings_from_text, client)
+                                                  async_get_openai_embeddings_from_text, client,
+                                                  _logprobs_of(completion.choices, consensus_settings))
     return _assemble_plain(completion, list(completion.choices), content, likelihoods)
 
 
@@ -290,8 +317,10 @@ def consolidate_parsed_chat_completions(
     if len(completion.choices) == 1:
         return KLLMsParsedChatCompletion.model_validate(completion.model_dump())
     _check_candidates(len(completion.choices))
-    content, likelihoods = (_consensus_of_choices_native(completion.choices, consensus_settings, get_openai_embeddings_from_text)
-                            or _consensus_sync(_contents_of(completion.choices), consensus_settings, get_openai_embeddings_from_text, client))
+    lps = _logprobs_of(completion.choices, consensus_settings)
+    content, likelihoods = (_consensus_of_choices_native(completion.choices, consensus_settings, get_openai_embeddings_from_text, lps)
+                            or _consensus_sync(_contents_of(completion.choices), consensus_settings, get_openai_embeddings_from_text, client,
+                                               lps))
     return _assemble_parsed(completion, content, likelihoods, response_format, keep_usage=True)
 
 
@@ -308,13 +337,14 @@ async def async_consolidate_parsed_chat_completions(
         return KLLMsParsedChatCompletion.model_validate(completion.model_dump())
     _check_candidates(len(completion.choices))
     content, likelihoods = await _consensus_async(_contents_of(completion.choices), consensus_settings,
-                                                  async_get_openai_embeddings_from_text, client)
+                                                  async_get_openai_embeddings_from_text, client,
+                                                  _logprobs_of(completion.choices, consensus_settings))
     return _assemble_parsed(completion, content, likelihoods, response_format, keep_usage=False)
 
 
 def consolidate_contents_batch(records: List[List[str]], consensus_settings: ConsensusSettings = ConsensusSettings(),
                                get_openai_embeddings_from_text: Optional[SYNC_GET_OPENAI_EMBEDDINGS_FROM_TEXT_TYPE] = None,
-                               client: Any = None, device: int = 0):
+                               client: Any = None, device: int = 0, logprobs: Optional[List[List[List[float]]]] = None):
     """Batched consolidation of raw contents (new; the reference has no batch dimension): for every record, the n
     `choice.message.content` strings in -> (consensus content string, likelihoods) out, exactly what the per-request
     functions above put into choices[0] and `likelihoods`.
@@ -323,10 +353,20 @@ def consolidate_contents_batch(records: List[List[str]], consensus_settings: Con
     the GPU as they are; scan / key sort / typing / encode / K1 + K2 / emit run there); records that path does not model
     (nested objects, lists, multi-word strings, escapes, ...) are consolidated by the native host path (H1: C++ parse /
     alignment pre-pass / encode / decode + K1/K2/K4) inside the same call, and what that declines too (a key mixing objects
-    with other types, string pairs that need the embeddings service, non-ASCII text, ...) takes the Python + GPU path."""
+    with other types, string pairs that need the embeddings service, non-ASCII text, ...) takes the Python + GPU path.
+
+    With consensus_settings.candidate_weighting == "likelihood", logprobs[r][c] = the token logprobs of records[r][c] (one sequence
+    per text, empty texts included: their logprobs are dropped with them).  The batch goes to the weighted device entry
+    (kc_consolidate_json_packed_weighted); what it declines takes the weighted Python + GPU path (there is no weighted host path)."""
     from .. import _native
     default_eps = (consensus_settings.rel_eps, consensus_settings.abs_eps)
     native: List[Any] = [None] * len(records)
+    weighted = consensus_settings.candidate_weighting == "likelihood"
+    if weighted:
+        if logprobs is None:
+            raise ValueError("candidate_weighting='likelihood' needs logprobs: one list of token logprobs per candidate text")
+        if len(logprobs) != len(records) or any(lp is None or len(lp) != len(texts) for lp, texts in zip(logprobs, records)):
+            raise ValueError("candidate_weighting='likelihood': logprobs must hold one sequence per candidate text of every record")
     if _native_settings(consensus_settings):
         by_n: dict = {}
         for i, texts in enumerate(records):
@@ -334,21 +374,23 @@ def consolidate_contents_batch(records: List[List[str]], consensus_settings: Con
                 by_n.setdefault(len(texts), []).append(i)
         for n, idxs in by_n.items():
             _check_candidates(n)
-            outs = _native_consolidate([records[i] for i in idxs], default_eps[0], default_eps[1], device)
+            outs = _native_consolidate([records[i] for i in idxs], default_eps[0], default_eps[1], device,
+                                       [logprobs[i] for i in idxs] if weighted else None)
             for i, o in zip(idxs, outs):
                 native[i] = o
     results = []
     embed = get_openai_embeddings_from_text if get_openai_embeddings_from_text is not None else (lambda texts: [[0.0] for _ in texts])
-    for texts, nat in zip(records, native):
+    for i, (texts, nat) in enumerate(zip(records, native)):
         if nat is not None:
             results.append((nat[0], json.loads(nat[1])))
             continue
         contents = [_safe_parse_content(t) for t in texts if t]
+        lps = check_candidate_logprobs(consensus_settings, [lp for t, lp in zip(texts, logprobs[i]) if t], len(contents)) if weighted else None
         _check_candidates(len(contents))
         if len(texts) == 1:  # a single choice is returned as it is (reference consolidation.py:85-87)
             results.append((texts[0], None))
             continue
         # one non-empty content among several choices still goes through consensus_values, like the per-request path
-        value, likelihoods = _consensus_sync(contents, consensus_settings, embed, client)
+        value, likelihoods = _consensus_sync(contents, consensus_settings, embed, client, lps)
         results.append((_format_consensus_content(value), likelihoods))
     return results
